@@ -2,11 +2,20 @@
 """bench.py -- headline benchmark of the B200-native NeRF-LOAM hot path (BASELINE.json metric):
 neural-SDF samples/s per mapping iteration on a synthetic 100k-ray KITTI-shape scan.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one full mapping iteration of bundle_adjust_frames' loop body on every ray of one scan per GPU:
 pose -> rays -> octree traversal -> inverse-CDF sampling -> embedding gather + trilinear -> 16-256-256-1 MLP
 -> SDF/free-space loss -> backward (decoder, embeddings, pose) -> Adam on all three.  Prints ONE JSON line.
+
+--dump-outputs DIR writes what the last of the K timed steps hands back to its caller -- the embedding table, decoder and pose
+after Adam, and the loss -- as DIR/<name>.npy, arrays whose shapes depend only on the arguments.  The timed steps start from the
+seeded problem as built, so two builds run with the same arguments can be compared output for output; what differs between two
+runs of one build is the order of float atomics within those K steps, which a mapping loop amplifies (the pose gradient is a sum
+of ~10^5 cancelling terms, and the pose moves the rays: the number of samples, hence the per-sample SDF, is not dumped because
+its length differs by a few samples in 775k from run to run).  Measured on a B200: with --steps 1 two runs give the same loss bit
+for bit and the same parameters up to one bf16 rounding step of the table; with --steps 20 the parameters agree to ~2e-3
+relative norm.
 """
 import argparse
 import json
@@ -30,6 +39,10 @@ FLOPS_PER_SAMPLE_MAP_DEC = 419328             # BASELINE.md: MLP fwd + bwd-data 
 ISSUED_TF32_FLOPS_PER_SAMPLE = 2 * (3 * 16 * 256 + 3 * 256 * 256 + 2 * 256 * 256 + 3 * 256 * 16 + 2 * 256 * 256 + 3 * 256 * 32)
 WORKLOAD = "synthetic 100k-ray KITTI-shape scan (64x1563 beams, 82.7k returns), single-scan 0.3 m map, " \
            "mapping iteration on ALL rays, decoder+embeddings+pose updated, Adam included"
+# untimed steps between the warm-up and the clock, so that clocks, allocator, NCCL channels and the two-stream pipeline reach
+# steady state (64 steps took ~100 ms on a B200).  A fixed count, not a duration: the state the timed steps start from must not
+# depend on how fast the machine is
+SETTLE_STEPS = 64
 
 
 def peaks():
@@ -165,13 +178,16 @@ def run_ours(args):
             state["opt_frozen"].step()
             return
         if state["opt"] is None:
-            groups = list(emb_group)
-            groups += [dict(param=p.data, grad=g, lr=LR[1], side=True) for p, g in zip(bufs.params, bufs.grads)]
-            groups += [dict(param=pose6[0], grad=eng.pose_grad[0], lr=LR[2])]
-            state["opt"] = nl.engine.FusedAdam(groups, ctl=lambda: eng.ctl)
+            state["opt"] = new_opt(emb_group)
         # pipelined: the decoder's Adam follows its weight-gradient kernels on the side stream; the main stream goes on with the
         # embedding / pose update and the next iteration's rays, traversal, sampling and gather, and joins before its decoder
         state["opt"].step(side_stream=eng.deferred_stream())
+
+    def new_opt(emb_group):
+        groups = list(emb_group)
+        groups += [dict(param=p.data, grad=g, lr=LR[1], side=True) for p, g in zip(bufs.params, bufs.grads)]
+        groups += [dict(param=pose6[0], grad=eng.pose_grad[0], lr=LR[2])]
+        return nl.engine.FusedAdam(groups, ctl=lambda: eng.ctl)
 
     def sync_all():
         if world > 1:
@@ -193,30 +209,33 @@ def run_ours(args):
         return a.elapsed_time(b)
 
     # ---------------- device-resident timing (value) ----------------
+    # the timed steps start from the problem as built, not from what the warm-up and settle steps left: those accumulate gradients
+    # with float atomics, so their result differs in the last bits from run to run, and Adam amplifies that step after step
+    start = [t.detach().clone() for t in [emb, pose6] + bufs.params]
     eng.begin_call()
     W = max(args.warmup, 3)
     for _ in range(W):
         step(d_dirs, d_gt, d_cos)
-    # settle: clocks, allocator, NCCL channels and the two-stream pipeline reach steady state before the clock starts (untimed, >= 100 ms)
-    sync_all()
-    t_s = time.perf_counter()
-    n_settle = 0
-    while time.perf_counter() - t_s < 0.10:
-        for _ in range(8):
-            step(d_dirs, d_gt, d_cos)
-        torch.cuda.synchronize()
-        n_settle += 8
-    if world > 1:       # same number of settle steps on every rank (collectives inside)
-        import torch.distributed as dist
-        t_n = torch.tensor([n_settle], device=dev); dist.all_reduce(t_n, op=dist.ReduceOp.MAX)
-        for _ in range(int(t_n.item()) - n_settle):
-            step(d_dirs, d_gt, d_cos)
-        n_settle = int(t_n.item())
+    for i in range(SETTLE_STEPS):
+        step(d_dirs, d_gt, d_cos)
+        if i % 8 == 7:
+            torch.cuda.synchronize()
+    eng.join_side()
+    sync_all()                                         # multi-GPU: no peer still reads this rank's table
+    with torch.no_grad():
+        for t, t0 in zip([emb, pose6] + bufs.params, start):
+            t.copy_(t0)
+        if peer is not None:
+            peer.m.zero_(); peer.v.zero_()
+    eng.begin_call()                                   # Adam's step count
+    state["opt"] = new_opt([] if peer is not None else [dict(param=emb, grad=eng.grad_emb, lr=LR[0])])
     l0 = nl._capi.LAUNCHES
     ms_total = timed(lambda: step(d_dirs, d_gt, d_cos), args.steps, eng.join_side)   # deferred decoder work of the last iteration is inside
     launches = nl._capi.LAUNCHES - l0
     st = eng.read_stats()
     n_local = st.n_samples
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, st, dec, emb, pose6)
     # ---------------- the same loop over >= 250 ms with one event per step: median / max (what a 32 ms window cannot show) ----------------
     n_long = max(args.steps, int(0.25 / max(ms_total / args.steps * 1e-3, 1e-6)) + 1)
     if world > 1:
@@ -354,7 +373,7 @@ def run_ours(args):
                                   "decoder-gradient all-reduce (NCCL, side stream)"),
                    "l2": "per-step working set (samples x ~2.2 KB activations+features) ~1.9 GB >> 126 MB L2; no flush needed",
                    "sampler_noise": "in-kernel counter RNG", "loss": loss_val,
-                   "untimed_before_clock": f"{W} warm-up steps + {n_settle} settle steps (>= 100 ms)",
+                   "untimed_before_clock": f"{W} warm-up steps + {SETTLE_STEPS} settle steps, then parameters and Adam state reset to the seeded start",
                    "kernel_error_bits_over_all_steps": ctl[nl._capi.CTL_ERROR], "skipped_steps": ctl[nl._capi.CTL_SKIPPED],
                    "multi_gpu_exchange": peer_info},
         "e2e": {"value": e2e, "unit": "samples/s", "h2d_bytes_per_step": int(R * 20 * world), "d2h_bytes_per_step": int(160 * world),
@@ -431,6 +450,17 @@ def run_ours(args):
     if world == 1 and not os.environ.get("NL_BENCH_SKIP_CPU"):
         out["cpu_baseline"] = best_cpu_baseline(n_rays=4096, iters=3)
     print(json.dumps(out))
+
+
+def dump_outputs(out_dir, st, dec, emb, pose6):
+    """What the last timed step hands back, as out_dir/<name>.npy: the embedding table, decoder and pose after its Adam step
+    (fp32) and its loss with the free-space and SDF parts (fp64); ~2 MB in all."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"embeddings": emb, "pose": pose6}
+    arrays.update({"decoder." + k: v for k, v in dec.state_dict().items()})
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([st.loss, st.fs_loss, st.sdf_loss], np.float64))
 
 
 def strong_scaling_block(nl, dev, rank, world, group, scan, ms, dec, steps, sync_all, timed, use_peer=False):
@@ -871,6 +901,7 @@ if __name__ == "__main__":
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     a = ap.parse_args()
     # stdout carries exactly one JSON line: while the benchmark runs, file descriptor 1 points at stderr, so that library
     # banners written with printf (NCCL prints its version there) cannot get in front of it

@@ -106,7 +106,11 @@ def reference_map_states(voxels, children, features, voxel_size, table_rows=None
         g = torch.Generator().manual_seed(seed)
         per_vertex = (torch.randn((n, 16), generator=g) * init_std).to(torch.bfloat16)
         emb = per_vertex[add].contiguous()
-    id2[add] = torch.arange(0, add.shape[0], dtype=torch.int).view(-1, 1)
+    # `add` repeats a vertex once per voxel that references it, so which of its rows the table keeps is unspecified (a racy
+    # index_put_ in the reference, and a multi-threaded one on the host here): pinned to the last, so that every process builds
+    # the same table and row-wise results recorded in one process hold in another
+    last = torch.full((id2.shape[0],), -1, dtype=torch.long).scatter_reduce_(0, add, torch.arange(add.shape[0]), reduce="amax")
+    id2[add] = last[add].int().view(-1, 1)
     centres.requires_grad_()
     return {"voxel_vertex_idx": features, "voxel_center_xyz": centres, "voxel_structure": structure,
             "voxel_vertex_emb": emb.to(device).requires_grad_(), "voxel_id2embedding_id": id2}

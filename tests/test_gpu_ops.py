@@ -1,13 +1,11 @@
 """GPU parity tests of the individual C-ABI ops against the oracle, the golden vectors produced by the
-executed reference, and (when oracle/_ref/grid was built) the compiled unmodified reference kernels."""
-import ctypes as C
-import os
-
+executed reference, and the outputs of the compiled unmodified reference kernels recorded on a B200
+(tests/golden/reference_gpu.npz, tests/golden/make_golden_gpu.py)."""
 import numpy as np
 import pytest
 import torch
 
-from util import bf16_from_bits, golden, product_map, ref_grid, load_decoder
+from util import bf16_from_bits, golden, product_map, load_decoder
 
 pytestmark = pytest.mark.gpu
 
@@ -49,20 +47,25 @@ def test_svo_intersect_vs_oracle_and_reference(nl, scene):
     assert np.array_equal(idx[0].cpu().numpy(), oi)                     # voxel ids: bit-exact, DFS order
     np.testing.assert_allclose(mn[0].cpu().numpy(), omn, rtol=2e-6, atol=1e-6)   # __fdividef vs 1.0f/x
     np.testing.assert_allclose(mx[0].cpu().numpy(), omx, rtol=2e-6, atol=1e-6)
-    g = ref_grid()
-    if g is not None:                                                   # the real reference kernel, same GPU
-        G = 4                                                           # its wrapper batches rays and replicates the octree
-        K = ro.shape[1] // G
-        rs = ro[:, :G * K].reshape(G, K, 3).contiguous()
-        rdd = rd[:, :G * K].reshape(G, K, 3).contiguous()
-        ri, rmn, rmx = g.svo_intersect(rs, rdd, pts.expand(G, -1, -1).contiguous(), ch.expand(G, -1, -1).contiguous(), vs, 20)
-        mi, mmn, mmx = nl.grid.svo_intersect(rs, rdd, pts.expand(G, -1, -1).contiguous(), ch.expand(G, -1, -1).contiguous(), vs, 20)
-        assert torch.equal(ri, mi) and torch.equal(rmn, mmn) and torch.equal(rmx, mmx)   # bit-exact incl. depths
+    # the real reference kernel on a B200, called the way its wrapper calls it (rays batched, octree replicated per batch)
+    r = golden("reference_gpu.npz")
+    mi, mmn, mmx = nl.grid.svo_intersect(*intersect_batched(ro, rd, pts, ch), vs, 20)
+    rows = torch.from_numpy(r["isect_rows"]).long()
+    for got, want in ((mi, r["isect_idx"]), (mmn, r["isect_min"]), (mmx, r["isect_max"])):
+        assert torch.equal(got.reshape(-1, 20)[rows].cpu(), torch.from_numpy(want))      # bit-exact incl. depths
 
 
-def test_inverse_cdf_sampling_vs_oracle_and_reference(nl, scene):
+def intersect_batched(ro, rd, pts, ch, G=4):
+    """svo_intersect's inputs as the reference's wrapper lays them out: rays in G batches, the octree replicated per batch."""
+    K = ro.shape[1] // G
+    rep = lambda a: a.expand(G, -1, -1).contiguous()
+    return ro[:, :G * K].reshape(G, K, 3).contiguous(), rd[:, :G * K].reshape(G, K, 3).contiguous(), rep(pts), rep(ch)
+
+
+def inverse_cdf_inputs(z):
+    """inverse_cdf_sampling's inputs for the hit rays of render.npz: [Gb, H/Gb, P] hits padded by repeating the first ray, seeded
+    noise, probabilities and step counts as the reference's ray_sample computes them."""
     from oracle import kernels as OK
-    z, m = scene
     hits = z["hits"]
     P = z["hit_idx"].shape[1]
     idx = z["hit_idx"][hits]; mn = z["hit_min"][hits]; mx = z["hit_max"][hits]
@@ -80,34 +83,39 @@ def test_inverse_cdf_sampling_vs_oracle_and_reference(nl, scene):
     noise = rng.uniform(0.001, 0.999, size=(Gb, H // Gb, S)).astype(np.float32)
     shp = (Gb, H // Gb, P)
     t = lambda a, s: torch.from_numpy(np.ascontiguousarray(a.reshape(s))).cuda()
-    args = (t(I, shp), t(A, shp), t(B, shp), torch.from_numpy(noise).cuda(), t(PR, shp), t(ST, (Gb, H // Gb)))
+    return t(I, shp), t(A, shp), t(B, shp), torch.from_numpy(noise).cuda(), t(PR, shp), t(ST, (Gb, H // Gb))
+
+
+def test_inverse_cdf_sampling_vs_oracle_and_reference(nl, scene):
+    from oracle import kernels as OK
+    z, m = scene
+    args = inverse_cdf_inputs(z)
+    Gb, Hb, P = args[0].shape
+    S = args[3].shape[-1]
     si, sd, sl = nl.grid.inverse_cdf_sampling(*args, -1.0)
-    oi = np.empty((Gb, H // Gb, S), np.int32); od = np.empty_like(oi, dtype=np.float32); ol = np.empty_like(od)
+    oi = np.empty((Gb, Hb, S), np.int32); od = np.empty_like(oi, dtype=np.float32); ol = np.empty_like(od)
     a = [np.ascontiguousarray(x.cpu().numpy()) for x in args]
-    OK.lib().nlo_inverse_cdf_sampling(Gb, H // Gb, P, S, -1.0, OK._p(a[0]), OK._p(a[1]), OK._p(a[2]), OK._p(a[3]), OK._p(a[4]),
+    OK.lib().nlo_inverse_cdf_sampling(Gb, Hb, P, S, -1.0, OK._p(a[0]), OK._p(a[1]), OK._p(a[2]), OK._p(a[3]), OK._p(a[4]),
                                       OK._p(a[5]), OK._p(oi), OK._p(od), OK._p(ol))
     assert np.array_equal(si.cpu().numpy(), oi)
     assert np.array_equal(sd.cpu().numpy(), od) and np.array_equal(sl.cpu().numpy(), ol)   # same fp ops incl. the FMA
-    g = ref_grid()
-    if g is not None:
-        ri, rd_, rl = g.inverse_cdf_sampling(*args, -1.0)
-        assert torch.equal(ri, si) and torch.equal(rd_, sd) and torch.equal(rl, sl)
+    r = golden("reference_gpu.npz")                                    # the compiled reference kernel on a B200
+    rows = torch.from_numpy(r["icdf_rows"]).long()
+    for got, want in ((si, r["icdf_idx"]), (sd, r["icdf_depth"]), (sl, r["icdf_dist"])):
+        assert torch.equal(got.reshape(Gb * Hb, S)[rows].cpu(), torch.from_numpy(want))
 
 
 def test_reference_grid_pins_the_oracle(nl, scene):
-    """The oracle's C restatement of the two CUDA kernels against the compiled reference itself."""
-    g = ref_grid()
-    if g is None:
-        pytest.skip("oracle/_ref/grid not built")
+    """The oracle's C restatement of the two CUDA kernels against the compiled reference itself (its outputs recorded on a B200
+    for the rays of tests/golden/reference_gpu.npz)."""
     from oracle import kernels as OK
     z, m = scene
     vs = float(z["voxel_size"])
-    ro = torch.from_numpy(z["rays_o"]).cuda()[None].contiguous()
-    rd = torch.from_numpy(z["rays_d"]).cuda()[None].contiguous()
-    ri, rmn, rmx = g.svo_intersect(ro, rd, m["centres"].cuda()[None].contiguous(), m["structure"].cuda()[None].contiguous(), vs, 20)
-    oi, omn, omx = OK.svo_intersect(z["rays_o"], z["rays_d"], m["centres"].numpy(), m["structure"].numpy(), vs, 20)
-    assert np.array_equal(ri[0].cpu().numpy(), oi)
-    np.testing.assert_allclose(rmn[0].cpu().numpy(), omn, rtol=2e-6, atol=1e-6)
+    r = golden("reference_gpu.npz")
+    rows = r["isect_rows"]
+    oi, omn, omx = OK.svo_intersect(z["rays_o"][rows], z["rays_d"][rows], m["centres"].numpy(), m["structure"].numpy(), vs, 20)
+    assert np.array_equal(r["isect_idx"], oi)
+    np.testing.assert_allclose(r["isect_min"], omn, rtol=2e-6, atol=1e-6)
 
 
 @pytest.mark.parametrize("width", [256, 32])

@@ -38,18 +38,6 @@ def product_map(vox, voxel_size, id2emb=None, emb_bits=None, device="cuda", grid
     return out
 
 
-def ref_grid():
-    """The compiled, unmodified reference `grid` extension (oracle/_ref/grid), or None when it was not built."""
-    p = os.path.join(ROOT, "oracle", "_ref", "grid", "grid_ref.so")
-    if not os.path.exists(p):
-        return None
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("grid_ref", p)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
-
-
 def load_decoder(z, prefix, device="cuda", width=256):
     import nerfloam_b200 as nl
     dec = nl.lidar.Decoder(depth=2, width=width, in_dim=16, skips=[], embedder="none", multires=0)
