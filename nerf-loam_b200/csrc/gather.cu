@@ -14,8 +14,6 @@
 //
 // Numerics follow render_helpers.py:65: p = (xyz - centre) / voxel_size + 0.5 with a true division;
 // corner k = 4*kx + 2*ky + kz; w_k = (ax * ay) * az with a = p or 1-p.
-#include <cstdlib>
-
 #include "nl_cuda.cuh"
 
 namespace {
@@ -85,10 +83,10 @@ __global__ void __launch_bounds__(128) k_gather_fwd(long long M_host, const int3
 }
 
 // Backward: autograd of the forward above w.r.t. the embedding rows (scatter-add) and xyz (-> pose).
-// MERGE: consecutive samples of a ray usually sit in the same voxel (step = voxel/2) and therefore scatter to the same 8
-// rows; lanes at even positions of such a run add their right neighbour's (already bf16-rounded) contributions with one
-// shuffle per value and issue the atomics for both, the odd lanes issue none: ~40 % fewer L2 atomics.
-template <int MERGE>   // 0: one atomic set per sample; 1: runs merged pairwise; 2: in groups of up to four
+// Consecutive samples of a ray usually sit in the same voxel (step = voxel/2) and therefore scatter to the same 8 rows.  Runs
+// of equal voxel ids inside a warp are merged in groups of up to four: lanes at even positions of a run add their right
+// neighbour's (already bf16-rounded) contributions with one shuffle per value, lanes at positions 0 mod 4 then add the pair
+// sum two lanes to their right and issue the atomics for the group, the other lanes issue none.
 __global__ void __launch_bounds__(128) k_gather_bwd(long long M_host, const int32_t *__restrict__ M_dev,
                                                      const float *__restrict__ xyz, const int32_t *__restrict__ vox,
                                                      const float *__restrict__ centres, const int32_t *__restrict__ vox2row,
@@ -132,20 +130,17 @@ __global__ void __launch_bounds__(128) k_gather_bwd(long long M_host, const int3
             g[8] = g2.x; g[9] = g2.y; g[10] = g2.z; g[11] = g2.w; g[12] = g3.x; g[13] = g3.y; g[14] = g3.z; g[15] = g3.w;
             t = tri_coords(xyz + i * 3, centres + (size_t)v * 3, voxel_size);
         }
-        // run structure inside the warp (MERGE): emitters = even positions of a run of equal voxel ids
+        // run structure inside the warp: emitters = positions 0 mod 4 of a run of equal voxel ids
         bool emit = true, take = false, take2 = false;
-        if (MERGE && grad_emb) {
+        if (grad_emb) {
             const int vprev = __shfl_up_sync(0xffffffffu, v, 1);
             const bool head = (lane == 0) || (vprev != v) || (v < 0);
             const unsigned hf = __ballot_sync(0xffffffffu, head);
             const int head_lane = 31 - __clz(hf & (0xffffffffu >> (31 - lane)));
             const int pos = lane - head_lane;
-            emit = (pos & 1) == 0;
-            take = emit && lane < 31 && !((hf >> (lane + 1)) & 1u);   // the right neighbour continues this run
-            if (MERGE == 2) {
-                emit = (pos & 3) == 0;
-                take2 = emit && lane < 30 && !((hf >> (lane + 1)) & 3u);   // so does the lane after it (which holds a pair sum)
-            }
+            take = (pos & 1) == 0 && lane < 31 && !((hf >> (lane + 1)) & 1u);   // the right neighbour continues this run
+            emit = (pos & 3) == 0;
+            take2 = emit && lane < 30 && !((hf >> (lane + 1)) & 3u);   // so does the lane after it (which holds a pair sum)
         }
         const float inv_vs = 1.0f / voxel_size;
 #pragma unroll
@@ -162,14 +157,10 @@ __global__ void __launch_bounds__(128) k_gather_bwd(long long M_host, const int3
                 for (int e = 0; e < 16; ++e) {
                     c[e] = has_row ? g[e] * w : 0.f;
                     if (round_bf16) c[e] = nl_round_bf16(c[e]);
-                    if (MERGE) {
-                        const float nb = __shfl_down_sync(0xffffffffu, c[e], 1);
-                        if (take) c[e] += nb;
-                    }
-                    if (MERGE == 2) {
-                        const float nb = __shfl_down_sync(0xffffffffu, c[e], 2);
-                        if (take2) c[e] += nb;
-                    }
+                    const float nb = __shfl_down_sync(0xffffffffu, c[e], 1);
+                    if (take) c[e] += nb;
+                    const float nb2 = __shfl_down_sync(0xffffffffu, c[e], 2);
+                    if (take2) c[e] += nb2;
                 }
                 if (has_row && emit) {
                     float4 *dst = reinterpret_cast<float4 *>(grad_emb + (size_t)rows[k] * 16);
@@ -267,16 +258,10 @@ extern "C" int nl_gather_trilinear_bwd(int64_t M, const int32_t *d_M_dev, const 
     if (pose_acc && (!s_ray || !s_depth || !ray_dir_local || n_frames <= 0 || n_frames > 1024))
         return nl_set_error("nl_gather_trilinear_bwd: pose accumulation needs s_ray, s_depth, ray_dir_local, 0 < n_frames <= 1024");
     const size_t smem = pose_acc ? sizeof(float) * 12 * (size_t)n_frames : 0;
-    static const int merge = [] { const char *e = getenv("NL_GATHER_MERGE"); return e ? atoi(e) : 2; }();
-#define NL_LAUNCH_GBWD(MG)                                                                                                          \
-    k_gather_bwd<MG><<<persistent_blocks(M, 128, 16), 128, smem, (cudaStream_t)stream>>>(                                          \
-        M, d_M_dev, xyz, vox, centres, vox2row, reinterpret_cast<const uint4 *>(emb), voxel_size,                                   \
-        reinterpret_cast<const float4 *>(dfeats), round_bf16, grad_emb, dxyz, s_ray, s_depth, ray_dir_local, ray_frame, n_frames,   \
-        pose_acc)
-    if (merge == 2) NL_LAUNCH_GBWD(2);
-    else if (merge == 1) NL_LAUNCH_GBWD(1);
-    else NL_LAUNCH_GBWD(0);
-#undef NL_LAUNCH_GBWD
+    k_gather_bwd<<<persistent_blocks(M, 128, 16), 128, smem, (cudaStream_t)stream>>>(
+        M, d_M_dev, xyz, vox, centres, vox2row, reinterpret_cast<const uint4 *>(emb), voxel_size,
+        reinterpret_cast<const float4 *>(dfeats), round_bf16, grad_emb, dxyz, s_ray, s_depth, ray_dir_local, ray_frame, n_frames,
+        pose_acc);
     NL_CHECK_LAUNCH("nl_gather_trilinear_bwd");
     return NL_OK;
 }

@@ -77,24 +77,6 @@ __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::
 __device__ __forceinline__ void tc_commit(uint32_t bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
-// the same arrive delivered to the barrier at this offset in BOTH CTAs of a 2-CTA cluster (weight stages shared by multicast)
-__device__ __forceinline__ void tc_commit_pair(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-                 "h"((uint16_t)3) : "memory");
-}
-// bulk copy global -> the same shared-memory offset of both CTAs of the pair; each CTA's barrier at `bar` receives the bytes
-__device__ __forceinline__ void bulk_g2s_pair(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(dst),
-                 "l"(src), "r"(bytes), "r"(bar), "h"((uint16_t)3) : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_cta_rank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
 
 // K-major SWIZZLE_128B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor): start>>4 [0,14), LBO>>4 [16,30)
 // (ignored for swizzled K-major, set to 1), SBO>>4 = 1024>>4 [32,46), version 1 [46,48), layout SWIZZLE_128B = 2 [61,64)
@@ -454,18 +436,13 @@ __device__ __forceinline__ void store_a_row_fast(uint32_t stage, const uint32_t 
 // Warp roles (NTHREADS_TRAIN = 320): warps 0-7 epilogue (group g = warp >> 2, TMEM lane quarter q = warp & 3), warp 8
 // producer, warp 9 MMA issuer + TMEM owner.  The two single-thread roles get the HIGHEST warp ids: the per-SMSP arbiter
 // prefers the highest warp id, so the busy epilogue warps cannot starve the thread that feeds the tensor core.
-// TS = true: the A operands of both backward GEMMs come from TMEM instead of shared memory.  The 0/1 mask of backward
-// layer 2 is written (tcgen05.st) over the dead layer-2 accumulator right where each thread read its pre-activations, so
-// those 8 K-blocks need no activation stage, no smem stores and no per-chunk hand-shake; the dh1 chunks of backward
-// layer 1 go through two 64-column TMEM slots (hi | lo), one per epilogue group.  Shared-memory traffic of those 16
-// steps drops to the weight panels, and the tiny N = 16 MMAs no longer fetch a 4 KB A tile from smem each.
-// PAIR = true (launched as clusters of 2 CTAs): the two CTAs of a pair walk through the SAME sequence of weight stages, each
-// on its own tile, so every stage is fetched from L2 once per pair -- CTA 0 loads the hi panel, CTA 1 the lo panel, each copy
-// multicast into both shared memories -- instead of once per CTA.  Backward layer 2 is bound by exactly that stream (64 KB per
-// K-block and SM, ~57 B/clk/SM, the L2's limit chip-wide); halving it is what moves it towards its tensor floor.  A stage is
-// refilled only when BOTH CTAs' MMAs have retired it (their tcgen05.commit is multicast to both b_empty barriers, count 2), and
-// both CTAs run the same number of rounds (a missing last tile is processed with all rows dead).
-template <bool WGRAD, bool TS, bool PAIR>
+// Only the forward steps 0..8 take their A operand from the shared-memory activation stages.  The A operands of both backward
+// GEMMs come from TMEM: the 0/1 mask of backward layer 2 is written (tcgen05.st) over the dead layer-2 accumulator right where
+// each thread read its pre-activations, so those 8 K-blocks need no activation stage, no smem stores and no per-chunk
+// hand-shake; the dh1 chunks of backward layer 1 go through two 64-column TMEM slots (hi | lo), one per epilogue group.
+// Shared-memory traffic of those 16 steps is the weight panels alone, and the tiny N = 16 MMAs fetch no A tile from smem.
+// Every CTA streams each weight stage from L2 itself; backward layer 2 is bound by that stream (64 KB per K-block and SM).
+template <bool WGRAD>
 __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams p) {
     extern __shared__ uint8_t smem_raw[];
     const uint32_t raw = smem_u32(smem_raw);
@@ -477,7 +454,7 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
     float *w2s = b1s + WN;
     uint64_t *bars = reinterpret_cast<uint64_t *>(sm + SMEM_DATA + 3 * WN * 4);
     // barriers: 0,1 b_full  2,3 b_empty  4,5 a_full  6,7 a_empty  8 d1_full  9 d2_full  10 d3_full  11 d4_full  12 d4_empty
-    //           TS: 14,15 slot_full[g]  16,17 slot_empty[g]  18..25 mask_full[K-block]
+    //           14,15 slot_full[g]  16,17 slot_empty[g]  18..25 mask_full[K-block]
     const uint32_t bar0 = smem_u32(bars);
     auto BAR = [&](int i) { return bar0 + 8u * i; };
     uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(bars + 28);
@@ -488,14 +465,11 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
 #define NL_STAMP(role, step, k) do { if (dbg && tl == 1 && (threadIdx.x & 31) == 0) dbg[((role) * 25 + (step)) * 8 + (k)] = clock64(); } while (0)
     const long long M = p.M_dev ? min((long long)*p.M_dev, p.M_host) : p.M_host;
     const long long ntiles = (M + TM - 1) / TM;
-    // tiles this CTA loops over: with PAIR every CTA runs the same number of rounds (tiles >= ntiles have only dead rows)
-    const long long nt_loop = PAIR ? ((ntiles + gridDim.x - 1) / gridDim.x) * gridDim.x : ntiles;
-    const uint32_t pair_rank = PAIR ? cluster_cta_rank() : 0u;
 
     for (int i = tid; i < WN; i += NTHREADS_TRAIN) { b0s[i] = p.b0[i]; b1s[i] = p.b1[i]; w2s[i] = p.w2[i]; }
     if (tid == 0) {
         mbar_init(BAR(0), 1); mbar_init(BAR(1), 1);
-        mbar_init(BAR(2), PAIR ? 2 : 1); mbar_init(BAR(3), PAIR ? 2 : 1);   // b_empty: the MMAs of both CTAs of a pair
+        mbar_init(BAR(2), 1); mbar_init(BAR(3), 1);
         mbar_init(BAR(4), 4); mbar_init(BAR(5), 4);      // a_full: the 4 warps of the group that owns the chunk
         mbar_init(BAR(6), 1); mbar_init(BAR(7), 1);
         mbar_init(BAR(8), 1); mbar_init(BAR(9), 1); mbar_init(BAR(10), 1); mbar_init(BAR(11), 1);
@@ -511,19 +485,18 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
     }
     tc_fence_before();
     __syncthreads();
-    if (PAIR) cluster_sync_all();                // the partner's barriers exist before any multicast copy / commit can reach them
     tc_fence_after();
     const uint32_t tmem = *tmem_slot;
     const uint32_t D1 = tmem, D2 = tmem + 256;   // D3 aliases D1, D4 aliases D2[0:16]
-    // TS: mask2 overwrites D2 (all 256 columns) for steps 9..16; dh1 slot g = D2[64 + 64g, +64) (hi | lo) for steps 17..24
+    // mask2 overwrites D2 (all 256 columns) for steps 9..16; dh1 slot g = D2[64 + 64g, +64) (hi | lo) for steps 17..24
     auto SLOT = [&](int g) { return D2 + 64u + 64u * (uint32_t)g; };
-    // activation-stage use index: without TS every step uses a stage, with TS only steps 0..8 of each tile do
-    auto AIT = [&](uint32_t tl, int step) { return TS ? tl * 9u + (uint32_t)step : tl * (uint32_t)STEPS_TRAIN + (uint32_t)step; };
+    // activation-stage use index: only steps 0..8 of each tile use a stage
+    auto AIT = [&](uint32_t tl, int step) { return tl * 9u + (uint32_t)step; };
 
     if (warp == 8) {
         // ===== producer (warp-uniform loop, one elected lane issues the copies) =====
         uint32_t it = 0, tl = 0;
-        for (long long tile = blockIdx.x; tile < nt_loop; tile += gridDim.x, ++tl) {
+        for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++tl) {
             for (int step = 0; step < STEPS_TRAIN; ++step, ++it) {
                 const uint32_t s = it & 1, ph = (it >> 1) & 1;
                 const uint32_t bytes = (step < 17) ? PANEL_B : PANEL_B16;
@@ -531,14 +504,10 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
                 mbar_wait(BAR(2 + s), ph ^ 1);
                 NL_STAMP(0, step, 1);
                 if (elect_one()) {
-                    mbar_expect_tx(BAR(0 + s), 2 * bytes);            // hi + lo land in this CTA whoever fetches them
+                    mbar_expect_tx(BAR(0 + s), 2 * bytes);            // hi + lo
                     const uint8_t *src = p.panels + (size_t)step * STAGE_B;
-                    if (PAIR) {                                       // this CTA fetches one of the two panels for both CTAs
-                        bulk_g2s_pair(sB + s * STAGE_B + pair_rank * PANEL_B, src + pair_rank * PANEL_B, bytes, BAR(0 + s));
-                    } else {
-                        bulk_g2s(sB + s * STAGE_B, src, bytes, BAR(0 + s));
-                        bulk_g2s(sB + s * STAGE_B + PANEL_B, src + PANEL_B, bytes, BAR(0 + s));
-                    }
+                    bulk_g2s(sB + s * STAGE_B, src, bytes, BAR(0 + s));
+                    bulk_g2s(sB + s * STAGE_B + PANEL_B, src + PANEL_B, bytes, BAR(0 + s));
                 }
                 __syncwarp();
             }
@@ -547,7 +516,7 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
         // ===== MMA issuer (warp-uniform loop, one elected lane issues) =====
         constexpr uint32_t idesc256 = make_idesc(TM, WN), idesc16 = make_idesc(TM, 16);
         uint32_t it = 0, tl = 0;
-        for (long long tile = blockIdx.x; tile < nt_loop; tile += gridDim.x, ++tl) {
+        for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++tl) {
             for (int step = 0; step < STEPS_TRAIN; ++step, ++it) {
                 const uint32_t s = it & 1, ph = (it >> 1) & 1;
                 NL_STAMP(1, step, 0);
@@ -555,7 +524,7 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
                 mbar_wait(BAR(0 + s), ph);
                 NL_STAMP(1, step, 1);
                 const uint32_t b_hi = sB + s * STAGE_B;
-                if (!TS || step <= 8) {
+                if (step <= 8) {
                     const uint32_t ai = AIT(tl, step), as = ai & 1, aph = (ai >> 1) & 1;
                     mbar_wait(BAR(4 + as), aph);
                     NL_STAMP(1, step, 2);
@@ -563,19 +532,14 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
                     const uint32_t a_hi = sA + as * STAGE_A;
                     if (elect_one()) {
                         if (step == 0) issue_kblock<2, 3>(D1, a_hi, b_hi, idesc256, 0u);                      // layer 1 (K = 16)
-                        else if (step <= 8) issue_kblock<4, 3>(D2, a_hi, b_hi, idesc256, step == 1 ? 0u : 1u);    // layer 2
-                        else if (step <= 16) issue_kblock<4, 2>(D1, a_hi, b_hi, idesc256, step == 9 ? 0u : 1u);   // backward layer 2: the 0/1
-                                                                                                                  // mask operand has no lo part
-                        else issue_kblock<4, 3>(D2, a_hi, b_hi, idesc16, step == 17 ? 0u : 1u);                   // backward layer 1 (N = 16)
-                        if (PAIR) tc_commit_pair(BAR(2 + s)); else tc_commit(BAR(2 + s));
+                        else issue_kblock<4, 3>(D2, a_hi, b_hi, idesc256, step == 1 ? 0u : 1u);               // layer 2
+                        tc_commit(BAR(2 + s));
                         tc_commit(BAR(6 + as));
                         if (step == 0) tc_commit(BAR(8));
                         if (step == 8) tc_commit(BAR(9));
-                        if (step == 16) tc_commit(BAR(10));
-                        if (step == 24) tc_commit(BAR(11));
                     }
                 } else if (step <= 16) {
-                    // ---- TS backward layer 2: A = mask2 columns of K-block jb in TMEM ----
+                    // ---- backward layer 2: A = mask2 columns of K-block jb in TMEM (0/1, exact in tf32: no lo term) ----
                     mbar_wait(BAR(18 + (step - 9)), tl & 1);
                     NL_STAMP(1, step, 2);
                     tc_fence_after();
@@ -591,11 +555,11 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
                                 acc = 1u;
                             }
                         }
-                        if (PAIR) tc_commit_pair(BAR(2 + s)); else tc_commit(BAR(2 + s));
+                        tc_commit(BAR(2 + s));
                         if (step == 16) tc_commit(BAR(10));
                     }
                 } else {
-                    // ---- TS backward layer 1: A = dh1 chunk (hi | lo) in the TMEM slot of the group that owns K-block kb ----
+                    // ---- backward layer 1 (N = 16): A = dh1 chunk (hi | lo) in the TMEM slot of the group that owns K-block kb ----
                     const int kb = step - 17, g = kb & 1;
                     const uint32_t u = tl * 4u + (uint32_t)(kb >> 1);
                     mbar_wait(BAR(14 + g), u & 1);
@@ -613,7 +577,7 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
                                 acc = 1u;
                             }
                         }
-                        if (PAIR) tc_commit_pair(BAR(2 + s)); else tc_commit(BAR(2 + s));
+                        tc_commit(BAR(2 + s));
                         tc_commit(BAR(16 + g));
                         if (step == 24) tc_commit(BAR(11));
                     }
@@ -663,15 +627,15 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
         };
         prefetch(blockIdx.x);
         uint32_t tl = 0;
-        for (long long tile = blockIdx.x; tile < nt_loop; tile += gridDim.x, ++tl) {
+        for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++tl) {
             const long long m = tile * TM + row;
             const bool live = m < M;
             const uint32_t fl = fl_n;
             const float z = z_n, dgt = dgt_n, dext = dext_n;
             uint32_t mask1[4], mask2[4];
-            // ---- step 0: x -> A (group 0).  With TS the activation stages are idle during the backward steps, so the next
-            // tile's x was already staged at the end of the previous tile (stage_x below) ----
-            if (g == 0 && (!TS || tl == 0)) {
+            // ---- step 0: x -> A (group 0).  The activation stages are idle during the backward steps, so every later tile's x
+            // is staged at the end of the tile before it (below) ----
+            if (g == 0 && tl == 0) {
                 const uint32_t it = AIT(tl, 0), s = it & 1, ph = (it >> 1) & 1;
                 if (WGRAD) { if (lane == 0) bulk_wait_read(); __syncwarp(); }
                 mbar_wait(BAR(6 + s), ph ^ 1);
@@ -718,7 +682,7 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
                 fence_proxy_async();
                 if (q == 0 && lane == 0) NL_STAMP(2 + g, 1 + kb, 7);
                 __syncwarp();
-                if (WGRAD && lane == 0 && tile < ntiles) bulk_s2g(p.act_h1 + ((size_t)(tile * 8 + kb) * TM + q * 32) * 32, sA + s * STAGE_A + q * 4096, 4096);
+                if (WGRAD && lane == 0) bulk_s2g(p.act_h1 + ((size_t)(tile * 8 + kb) * TM + q * 32) * 32, sA + s * STAGE_A + q * 4096, 4096);
                 if (lane == 0) mbar_arrive(BAR(4 + s));
                 if (q == 0 && lane == 0) NL_STAMP(2 + g, 1 + kb, 3);
             }
@@ -741,16 +705,15 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
                     const bool on = t > 0.f;
                     mk |= on ? (1u << i) : 0u;
                     acc4[i & 3] = fmaf(on ? t : 0.f, w2s[cb * 32 + i], acc4[i & 3]);
-                    if (TS) v[i] = on ? 0x3f800000u : 0u;       // 1.0f / 0.0f: the A operand of backward layer 2
+                    v[i] = on ? 0x3f800000u : 0u;               // 1.0f / 0.0f: the A operand of backward layer 2
                 }
                 mask2[kk] = mk;
-                if (TS) {   // same lanes / columns this thread just read; backward layer 2 may start on this K-block right away
-                    tmem_st32(D2 + lane_addr + cb * 32, v);
-                    tmem_wait_st();
-                    tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(BAR(18 + cb));
-                }
+                // same lanes / columns this thread just read; backward layer 2 may start on this K-block right away
+                tmem_st32(D2 + lane_addr + cb * 32, v);
+                tmem_wait_st();
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive(BAR(18 + cb));
             }
             float *part = sdf_part + (tl & 1) * 256;
             part[g * 128 + row] = (acc4[0] + acc4[1]) + (acc4[2] + acc4[3]);
@@ -776,35 +739,14 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
                     }
                 }
             }
-            if (WGRAD && tile < ntiles) {            // (PAIR: a padding tile beyond the data has no panel rows)
+            if (WGRAD) {
                 if (g == 0) {
                     gb2r += dsdf;
                     p.act_dsdf[tile * TM + row] = dsdf;
                 }
                 *reinterpret_cast<uint4 *>(p.act_mask2 + (size_t)(tile * TM + row) * 8 + g * 4) = make_uint4(mask2[0], mask2[1], mask2[2], mask2[3]);
             }
-            // ---- steps 9..16: the 0/1 mask chunks as activation stages (TS: already in TMEM) ----
-#pragma unroll 1
-            for (int kk = 0; kk < (TS ? 0 : 4); ++kk) {
-                const int jb = 2 * kk + g;
-                const uint32_t it = AIT(tl, 9 + jb), s = it & 1, ph = (it >> 1) & 1;
-                if (q == 0 && lane == 0) NL_STAMP(2 + g, 9 + jb, 0);
-                if (WGRAD) { if (lane == 0) bulk_wait_read(); __syncwarp(); }
-                if (q == 0 && lane == 0) NL_STAMP(2 + g, 9 + jb, 1);
-                mbar_wait(BAR(6 + s), ph ^ 1);
-                if (q == 0 && lane == 0) NL_STAMP(2 + g, 9 + jb, 2);
-                {   // A = relu'(h2) as exact 0/1 tf32 values; dsdf and w2 are folded into the epilogue / the weight panels
-                    const uint32_t mk = mask2[kk], dst = sA + s * STAGE_A;
-#pragma unroll
-                    for (int c = 0; c < 8; ++c)
-                        st_shared_v4(dst + offc[c], (mk >> (4 * c)) & 1u ? 1.f : 0.f, (mk >> (4 * c + 1)) & 1u ? 1.f : 0.f,
-                                     (mk >> (4 * c + 2)) & 1u ? 1.f : 0.f, (mk >> (4 * c + 3)) & 1u ? 1.f : 0.f);
-                }
-                fence_proxy_async();
-                __syncwarp();
-                if (lane == 0) mbar_arrive(BAR(4 + s));
-                if (q == 0 && lane == 0) NL_STAMP(2 + g, 9 + jb, 3);
-            }
+            // steps 9..16 (backward layer 2) need nothing more from the epilogue: their 0/1 mask operand is already in TMEM
             prefetch(tile + gridDim.x);                 // next tile's x / loss inputs: a whole backward pass to arrive
             // ---- steps 17..24: dh1 (masked) chunks from D3 ----
             mbar_wait(BAR(10), tl & 1);
@@ -819,42 +761,30 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
 #pragma unroll
                 for (int i = 0; i < 32; ++i) h[i] = ((mask1[kk] >> i) & 1u) ? dsdf * __uint_as_float(v[i]) : 0.f;
                 if (q == 0 && lane == 0) NL_STAMP(2 + g, 17 + kb, 1);
-                if (TS) {
-                    // hi = the fp32 bits (the tensor core truncates to tf32), lo = x - trunc(x) rounded to tf32 (tf32_lo_part); both into this group's TMEM slot
-                    const uint32_t u = tl * 4u + (uint32_t)kk;
-                    mbar_wait(BAR(16 + g), (u & 1) ^ 1);               // the MMAs of this group's previous chunk retired
-                    if (q == 0 && lane == 0) NL_STAMP(2 + g, 17 + kb, 2);
-                    uint32_t w[32];
+                // hi = the fp32 bits (the tensor core truncates to tf32), lo = x - trunc(x) rounded to tf32 (tf32_lo_part); both into this group's TMEM slot
+                const uint32_t u = tl * 4u + (uint32_t)kk;
+                mbar_wait(BAR(16 + g), (u & 1) ^ 1);               // the MMAs of this group's previous chunk retired
+                if (q == 0 && lane == 0) NL_STAMP(2 + g, 17 + kb, 2);
+                uint32_t w[32];
 #pragma unroll
-                    for (int i = 0; i < 32; ++i) w[i] = __float_as_uint(h[i]);
-                    tmem_st32(SLOT(g) + lane_addr, w);
+                for (int i = 0; i < 32; ++i) w[i] = __float_as_uint(h[i]);
+                tmem_st32(SLOT(g) + lane_addr, w);
 #pragma unroll
-                    for (int i = 0; i < 32; ++i) w[i] = __float_as_uint(tf32_lo_part(h[i]));
-                    tmem_st32(SLOT(g) + lane_addr + 32, w);
-                    tmem_wait_st();
-                    tc_fence_before();
+                for (int i = 0; i < 32; ++i) w[i] = __float_as_uint(tf32_lo_part(h[i]));
+                tmem_st32(SLOT(g) + lane_addr + 32, w);
+                tmem_wait_st();
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive(BAR(14 + g));
+                if (WGRAD) {   // panel store for gW0 / gb0: staged through the activation stage this group used in steps 1..8
+                    const uint32_t sg = sA + ((tl + 1u + (uint32_t)g) & 1u) * STAGE_A;
+                    if (lane == 0) bulk_wait_read();
                     __syncwarp();
-                    if (lane == 0) mbar_arrive(BAR(14 + g));
-                    if (WGRAD) {   // panel store for gW0 / gb0: staged through the activation stage this group used in steps 1..8
-                        const uint32_t sg = sA + ((tl + 1u + (uint32_t)g) & 1u) * STAGE_A;
-                        if (lane == 0) bulk_wait_read();
-                        __syncwarp();
 #pragma unroll
-                        for (int c = 0; c < 8; ++c) st_shared_v4(sg + offc[c], h[c * 4], h[c * 4 + 1], h[c * 4 + 2], h[c * 4 + 3]);
-                        fence_proxy_async();
-                        __syncwarp();
-                        if (lane == 0 && tile < ntiles) bulk_s2g(p.act_dh1 + ((size_t)(tile * 8 + kb) * TM + q * 32) * 32, sg + q * 4096, 4096);
-                    }
-                } else {
-                    const uint32_t it = AIT(tl, 17 + kb), s = it & 1, ph = (it >> 1) & 1;
-                    if (WGRAD) { if (lane == 0) bulk_wait_read(); __syncwarp(); }
-                    mbar_wait(BAR(6 + s), ph ^ 1);
-                    if (q == 0 && lane == 0) NL_STAMP(2 + g, 17 + kb, 2);
-                    store_a_row_fast(sA + s * STAGE_A, offc, h);
+                    for (int c = 0; c < 8; ++c) st_shared_v4(sg + offc[c], h[c * 4], h[c * 4 + 1], h[c * 4 + 2], h[c * 4 + 3]);
                     fence_proxy_async();
                     __syncwarp();
-                    if (WGRAD && lane == 0 && tile < ntiles) bulk_s2g(p.act_dh1 + ((size_t)(tile * 8 + kb) * TM + q * 32) * 32, sA + s * STAGE_A + q * 4096, 4096);
-                    if (lane == 0) mbar_arrive(BAR(4 + s));
+                    if (lane == 0) bulk_s2g(p.act_dh1 + ((size_t)(tile * 8 + kb) * TM + q * 32) * 32, sg + q * 4096, 4096);
                 }
                 if (q == 0 && lane == 0) NL_STAMP(2 + g, 17 + kb, 3);
             }
@@ -862,9 +792,9 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
                 if (lane == 0) bulk_wait_read();
                 asm volatile("bar.sync 2, 256;" ::: "memory");
             }
-            if (TS && g == 0 && tile + gridDim.x < nt_loop) {
-                // x of the next tile (prefetched above) -> its activation stage now: the MMA warp can issue the next layer 1
-                // right behind this tile's last backward MMAs instead of waiting for the d x read-back below
+            // x of the next tile (prefetched above) -> its activation stage now: the MMA warp can issue the next layer 1
+            // right behind this tile's last backward MMAs instead of waiting for the d x read-back below
+            if (g == 0 && tile + gridDim.x < ntiles) {
                 const uint32_t it = AIT(tl + 1, 0), s = it & 1, ph = (it >> 1) & 1;
                 if (WGRAD) { if (lane == 0) bulk_wait_read(); __syncwarp(); }
                 mbar_wait(BAR(6 + s), ph ^ 1);
@@ -916,31 +846,10 @@ __global__ void __launch_bounds__(NTHREADS_TRAIN, 1) k_mlp_tc_train(TrainParams 
     }
     tc_fence_before();
     __syncthreads();
-    if (PAIR) cluster_sync_all();                // neither CTA leaves while the other may still multicast into it
     if (warp == 9) {
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512u) : "memory");
     }
-}
-
-// launch as clusters of two CTAs (even grid, at most one CTA per SM)
-template <class K>
-int launch_pair(K kernel, int grid, int sms, const TrainParams &p, cudaStream_t stream) {
-    grid = (grid + 1) & ~1;
-    if (grid > (sms & ~1)) grid = sms & ~1;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid, 1, 1);
-    cfg.blockDim = dim3(NTHREADS_TRAIN, 1, 1);
-    cfg.dynamicSmemBytes = SMEM_TOTAL;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, p);
-    if (e != cudaSuccess) return nl_set_error_code(NL_ERR_CUDA, cudaGetErrorString(e));
-    return NL_OK;
 }
 
 // ================================================================================================
@@ -951,9 +860,10 @@ int launch_pair(K kernel, int grid, int sms, const TrainParams &p, cudaStream_t 
 //                                            h2 = m2 * (h1 . W1^T + b1), c[j] = sum_s m2[s][j] d[s])
 //   K = samples, streamed in K-blocks of 16 rows.  Both operands are MN-major (SWIZZLE_128B_BASE32B, the only layout
 //   tcgen05 takes for MN-major tf32).  Per K-block the producer bulk-copies the 16 rows of the h1 panels (16 KB, the
-//   K-major image k_mlp_tc_train stored), 512 B of mask bits and 64 B of dsdf; 4 converter warps expand the bits into
+//   K-major image k_mlp_tc_train stored), 512 B of mask bits and 64 B of dsdf; 8 converter warps expand the bits into
 //   the 0/1 A operand (exact in tf32: one term fewer than 3xTF32) and write hi/lo of d*h1 as the B operand.
-//   3-deep raw ring (17 KB) + 2-deep converted ring (48 KB).  Every CTA finally adds its partial sums with atomics.
+//   4-deep raw ring (17 KB stages) + 3-deep converted ring (48 KB stages), 219 KB of shared memory.  Every CTA finally adds
+//   its partial sums with atomics.
 // ================================================================================================
 constexpr int DW_KROWS = 16;
 constexpr int DW_PANEL = DW_KROWS * 128;        // 2 KB: 16 sample rows x 128 B
@@ -961,9 +871,11 @@ constexpr int DW_OPER = 8 * DW_PANEL;           // 16 KB: all 256 columns of one
 constexpr int DW_BITS = DW_KROWS * 32;          // 512 B of relu'(h2) bits
 constexpr int DW_RAW = DW_OPER + 1024;          // h1 raw (K-major SWIZZLE_128B image as stored in HBM) | bits | dsdf
 constexpr int DW_CONV = 3 * DW_OPER;            // 48 KB: A mask | B hi | B lo (MN-major SWIZZLE_128B_BASE32B)
-// ring depths are kept small enough (149 KB / 161 KB of shared memory) that blocks of other kernels -- the next iteration's
-// traversal needs 48 KB -- can share the SM with these persistent CTAs when the engine pipelines iterations
-constexpr int dw_smem(int nraw, int nconv) { return nraw * DW_RAW + nconv * DW_CONV + 1024 + 1024; }
+constexpr int DW_NCW = 8;                       // converter warps of k_dw1_tc and k_dw0_tc (warps 2..9)
+constexpr int DW_NCT = 32 * DW_NCW;             // converter threads
+constexpr int DW_THREADS = 64 + DW_NCT;         // + producer warp and MMA warp
+constexpr int DW_NRAW = 4, DW_NCONV = 3;        // ring depths of k_dw1_tc
+constexpr int DW_SMEM = DW_NRAW * DW_RAW + DW_NCONV * DW_CONV + 1024 + 1024;
 
 // MN-major SWIZZLE_128B_BASE32B descriptor (layout type 1): LBO = byte stride between 32-element MN groups (= one 2 KB
 // panel), SBO = byte stride between groups of 4 K rows (512 B); one k-step (K = 8) spans two such groups
@@ -971,11 +883,11 @@ __device__ __forceinline__ uint64_t make_desc_mn(uint32_t saddr) {
     return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)(DW_PANEL >> 4) << 16) | (32ull << 32) | (1ull << 46) | (1ull << 61);
 }
 
-template <int NCW, int NRAW, int NCONV>   // converter warps (4 or 8), ring depths
-__global__ void __launch_bounds__(64 + 32 * NCW, 1) k_dw1_tc(long long M_host, const int32_t *__restrict__ M_dev, const uint32_t *__restrict__ act_mask2,
-                                                         const float *__restrict__ act_dsdf, const float *__restrict__ act_h1,
-                                                         const float *__restrict__ W1, const float *__restrict__ w2, float *__restrict__ gW1,
-                                                         float *__restrict__ gW2) {
+__global__ void __launch_bounds__(DW_THREADS, 1) k_dw1_tc(long long M_host, const int32_t *__restrict__ M_dev, const uint32_t *__restrict__ act_mask2,
+                                                       const float *__restrict__ act_dsdf, const float *__restrict__ act_h1,
+                                                       const float *__restrict__ W1, const float *__restrict__ w2, float *__restrict__ gW1,
+                                                       float *__restrict__ gW2) {
+    constexpr int NRAW = DW_NRAW, NCONV = DW_NCONV;
     extern __shared__ uint8_t smem_raw[];
     const uint32_t raw = smem_u32(smem_raw);
     const uint32_t base = (raw + 1023u) & ~1023u;
@@ -992,8 +904,8 @@ __global__ void __launch_bounds__(64 + 32 * NCW, 1) k_dw1_tc(long long M_host, c
     const long long M = M_dev ? min((long long)*M_dev, M_host) : M_host;
     const long long nkb = ((M + TM - 1) / TM) * (TM / DW_KROWS);   // K-blocks of 16 rows (whole tiles: padded rows have dsdf = 0)
     if (tid == 0) {
-        for (int i = 0; i < NRAW; ++i) { mbar_init(BAR(i), 1); mbar_init(BAR(4 + i), NCW); }
-        for (int i = 0; i < NCONV; ++i) { mbar_init(BAR(8 + i), NCW); mbar_init(BAR(11 + i), 1); }
+        for (int i = 0; i < NRAW; ++i) { mbar_init(BAR(i), 1); mbar_init(BAR(4 + i), DW_NCW); }
+        for (int i = 0; i < NCONV; ++i) { mbar_init(BAR(8 + i), DW_NCW); mbar_init(BAR(11 + i), 1); }
         mbar_init(BAR(14), 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -1058,10 +970,10 @@ __global__ void __launch_bounds__(64 + 32 * NCW, 1) k_dw1_tc(long long M_host, c
             __syncwarp();
         }
     } else {
-        // converters (128 threads).  Stored h1 image: K-major SWIZZLE_128B (16 B chunk c of row r at c ^ (r & 7)); operand
+        // converters (256 threads).  Stored h1 image: K-major SWIZZLE_128B (16 B chunk c of row r at c ^ (r & 7)); operand
         // tiles: MN-major SWIZZLE_128B_BASE32B (32 B chunk c of row r at c ^ (r & 3)).  hi = the fp32 bits of d*h1
         // (truncated to tf32 by the hardware), lo = tf32(x - trunc(x)).
-        constexpr int NCT = 32 * NCW;                              // converter threads
+        constexpr int NCT = DW_NCT;
         const int ct = tid - 64;
         // mask expansion: one (column block, sample row) per group of NCT/128 threads, 8 / (NCT/128) float4 each
         constexpr int MSPLIT = NCT / 128;
@@ -1119,31 +1031,28 @@ __global__ void __launch_bounds__(64 + 32 * NCW, 1) k_dw1_tc(long long M_host, c
             tc_fence_after();
             const int q = warp & 3;
             const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-            // all CTAs finish at about the same time: start each one at a different (accumulator, column block) so the
-            // 148 partial sums do not hammer the same L2 lines simultaneously.  With 8 converter warps each accumulator
-            // half is drained by its own 4 warps.
-            for (int jj = 0; jj < (NCW == 8 ? 1 : 2); ++jj) {
-                const int jt = NCW == 8 ? ((warp - 2) >> 2) : ((jj + (blockIdx.x >> 3)) & 1);
-                const int j = jt * 128 + q * 32 + lane;
-                const float w2j = w2[j];
-                float dot = 0.f;
-                for (int cc = 0; cc < 8; ++cc) {
-                    const int cb = (cc + blockIdx.x) & 7;
-                    uint32_t v[32];
-                    tmem_ld32(tmem + lane_addr + jt * 256 + cb * 32, v);
-                    float4 *o = reinterpret_cast<float4 *>(gW1 + (size_t)j * WN + cb * 32);
-                    const float4 *wr = reinterpret_cast<const float4 *>(W1 + (size_t)j * WN + cb * 32);
+            // each accumulator half is drained by its own 4 converter warps.  All CTAs finish at about the same time: start
+            // each one at a different column block so the 148 partial sums do not hammer the same L2 lines simultaneously.
+            const int jt = (warp - 2) >> 2;
+            const int j = jt * 128 + q * 32 + lane;
+            const float w2j = w2[j];
+            float dot = 0.f;
+            for (int cc = 0; cc < 8; ++cc) {
+                const int cb = (cc + blockIdx.x) & 7;
+                uint32_t v[32];
+                tmem_ld32(tmem + lane_addr + jt * 256 + cb * 32, v);
+                float4 *o = reinterpret_cast<float4 *>(gW1 + (size_t)j * WN + cb * 32);
+                const float4 *wr = reinterpret_cast<const float4 *>(W1 + (size_t)j * WN + cb * 32);
 #pragma unroll
-                    for (int c = 0; c < 8; ++c) {
-                        const float4 w = wr[c];
-                        const float g0 = __uint_as_float(v[c * 4]), g1 = __uint_as_float(v[c * 4 + 1]), g2 = __uint_as_float(v[c * 4 + 2]),
-                                    g3 = __uint_as_float(v[c * 4 + 3]);
-                        dot = fmaf(w.x, g0, fmaf(w.y, g1, fmaf(w.z, g2, fmaf(w.w, g3, dot))));
-                        atomicAdd(o + c, make_float4(w2j * g0, w2j * g1, w2j * g2, w2j * g3));
-                    }
+                for (int c = 0; c < 8; ++c) {
+                    const float4 w = wr[c];
+                    const float g0 = __uint_as_float(v[c * 4]), g1 = __uint_as_float(v[c * 4 + 1]), g2 = __uint_as_float(v[c * 4 + 2]),
+                                g3 = __uint_as_float(v[c * 4 + 3]);
+                    dot = fmaf(w.x, g0, fmaf(w.y, g1, fmaf(w.z, g2, fmaf(w.w, g3, dot))));
+                    atomicAdd(o + c, make_float4(w2j * g0, w2j * g1, w2j * g2, w2j * g3));
                 }
-                atomicAdd(gW2 + j, dot);
             }
+            atomicAdd(gW2 + j, dot);
         }
     }
     tc_fence_before();
@@ -1162,11 +1071,12 @@ __global__ void __launch_bounds__(64 + 32 * NCW, 1) k_dw1_tc(long long M_host, c
 // ================================================================================================
 constexpr int D0_RAW = DW_OPER + 1024;          // dh1 raw (16 KB) | x rows (16 x 64 B)
 constexpr int D0_CONV = 2 * DW_OPER + 2 * DW_PANEL;   // A hi | A lo | B hi | B lo = 36 KB
-constexpr int d0_smem(int nraw, int nconv) { return nraw * D0_RAW + nconv * D0_CONV + 1024 + 1024; }
+constexpr int D0_NRAW = 4, D0_NCONV = 4;        // ring depths: 219 KB of shared memory
+constexpr int D0_SMEM = D0_NRAW * D0_RAW + D0_NCONV * D0_CONV + 1024 + 1024;
 
-template <int NCW, int NRAW, int NCONV>
-__global__ void __launch_bounds__(64 + 32 * NCW, 1) k_dw0_tc(long long M_host, const int32_t *__restrict__ M_dev, const float *__restrict__ act_dh1,
-                                                         const float *__restrict__ feats, float *__restrict__ gW0, float *__restrict__ gb0) {
+__global__ void __launch_bounds__(DW_THREADS, 1) k_dw0_tc(long long M_host, const int32_t *__restrict__ M_dev, const float *__restrict__ act_dh1,
+                                                       const float *__restrict__ feats, float *__restrict__ gW0, float *__restrict__ gb0) {
+    constexpr int NRAW = D0_NRAW, NCONV = D0_NCONV;
     extern __shared__ uint8_t smem_raw[];
     const uint32_t raw = smem_u32(smem_raw);
     const uint32_t base = (raw + 1023u) & ~1023u;
@@ -1182,8 +1092,8 @@ __global__ void __launch_bounds__(64 + 32 * NCW, 1) k_dw0_tc(long long M_host, c
     const long long M = M_dev ? min((long long)*M_dev, M_host) : M_host;
     const long long nkb = ((M + TM - 1) / TM) * (TM / DW_KROWS);
     if (tid == 0) {
-        for (int i = 0; i < NRAW; ++i) { mbar_init(BAR(i), 1); mbar_init(BAR(4 + i), NCW); }
-        for (int i = 0; i < NCONV; ++i) { mbar_init(BAR(8 + i), NCW); mbar_init(BAR(12 + i), 1); }
+        for (int i = 0; i < NRAW; ++i) { mbar_init(BAR(i), 1); mbar_init(BAR(4 + i), DW_NCW); }
+        for (int i = 0; i < NCONV; ++i) { mbar_init(BAR(8 + i), DW_NCW); mbar_init(BAR(12 + i), 1); }
         mbar_init(BAR(16), 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -1282,7 +1192,7 @@ __global__ void __launch_bounds__(64 + 32 * NCW, 1) k_dw0_tc(long long M_host, c
                 bl[o] = l;
             }
 #pragma unroll 4
-            for (int f = ct; f < DW_OPER / 16; f += 32 * NCW) {
+            for (int f = ct; f < DW_OPER / 16; f += DW_NCT) {
                 const int pnl = f >> 7, lr = (f >> 3) & 15, p16 = f & 7;
                 const int c16 = p16 ^ (lr & 7);
                 const int d16 = (((c16 >> 1) ^ (lr & 3)) << 1) | (c16 & 1);
@@ -1305,18 +1215,16 @@ __global__ void __launch_bounds__(64 + 32 * NCW, 1) k_dw0_tc(long long M_host, c
             tc_fence_after();
             const int q = warp & 3;
             const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-            for (int jj = 0; jj < (NCW == 8 ? 1 : 2); ++jj) {
-                const int jt = NCW == 8 ? ((warp - 2) >> 2) : ((jj + (blockIdx.x >> 3)) & 1);
-                const int k = jt * 128 + q * 32 + lane;
-                uint32_t v[32];
-                tmem_ld32(tmem + lane_addr + jt * 32, v);
-                float4 *o = reinterpret_cast<float4 *>(gW0 + (size_t)k * 16);
+            const int jt = (warp - 2) >> 2;             // each accumulator half is drained by its own 4 converter warps
+            const int k = jt * 128 + q * 32 + lane;
+            uint32_t v[32];
+            tmem_ld32(tmem + lane_addr + jt * 32, v);
+            float4 *o = reinterpret_cast<float4 *>(gW0 + (size_t)k * 16);
 #pragma unroll
-                for (int c = 0; c < 4; ++c)
-                    atomicAdd(o + c, make_float4(__uint_as_float(v[c * 4]), __uint_as_float(v[c * 4 + 1]), __uint_as_float(v[c * 4 + 2]),
-                                                 __uint_as_float(v[c * 4 + 3])));
-                atomicAdd(gb0 + k, __uint_as_float(v[16]));
-            }
+            for (int c = 0; c < 4; ++c)
+                atomicAdd(o + c, make_float4(__uint_as_float(v[c * 4]), __uint_as_float(v[c * 4 + 1]), __uint_as_float(v[c * 4 + 2]),
+                                             __uint_as_float(v[c * 4 + 3])));
+            atomicAdd(gb0 + k, __uint_as_float(v[16]));
         }
     }
     tc_fence_before();
@@ -1416,25 +1324,15 @@ extern "C" int nl_mlp_tc_train(int64_t M, const int32_t *d_M_dev, const float *f
     static std::mutex dev_mu;
     static bool configured_dev[NL_MAX_DEV] = {};
     static cudaEvent_t ev_dev[NL_MAX_DEV] = {};
-    static cudaStream_t s2_dev[NL_MAX_DEV] = {};                    // internal stream of k_dw0_tc when the two weight-gradient kernels run side by side
-    static cudaEvent_t e2_dev[NL_MAX_DEV] = {}, e3_dev[NL_MAX_DEV] = {};
     int cur_dev = 0;
     if (cudaGetDevice(&cur_dev) != cudaSuccess || cur_dev < 0 || cur_dev >= NL_MAX_DEV) return nl_set_error_code(NL_ERR_CUDA, "nl_mlp_tc_train: cudaGetDevice");
     std::lock_guard<std::mutex> dev_lock(dev_mu);
     bool &configured = configured_dev[cur_dev];
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(tc::k_mlp_tc_train<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_TOTAL);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::k_mlp_tc_train<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_TOTAL);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::k_mlp_tc_train<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_TOTAL);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::k_mlp_tc_train<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_TOTAL);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::k_mlp_tc_train<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_TOTAL);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::k_mlp_tc_train<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_TOTAL);
-#define NL_DW_ATTR(K, NR, NC, SM)                                                                                               \
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::K<4, NR, NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SM(NR, NC)); \
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::K<8, NR, NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SM(NR, NC));
-        NL_DW_ATTR(k_dw1_tc, 4, 3, dw_smem) NL_DW_ATTR(k_dw1_tc, 3, 3, dw_smem) NL_DW_ATTR(k_dw1_tc, 3, 2, dw_smem)
-        NL_DW_ATTR(k_dw0_tc, 4, 4, d0_smem) NL_DW_ATTR(k_dw0_tc, 4, 3, d0_smem) NL_DW_ATTR(k_dw0_tc, 3, 3, d0_smem)
-#undef NL_DW_ATTR
+        cudaError_t e = cudaFuncSetAttribute(tc::k_mlp_tc_train<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_TOTAL);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::k_mlp_tc_train<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::SMEM_TOTAL);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::k_dw1_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::DW_SMEM);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc::k_dw0_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::D0_SMEM);
         if (e != cudaSuccess) return nl_set_error_code(NL_ERR_CUDA, cudaGetErrorString(e));
         configured = true;
     }
@@ -1445,18 +1343,10 @@ extern "C" int nl_mlp_tc_train(int64_t M, const int32_t *d_M_dev, const float *f
     p.truncation = truncation; p.dsdf_ext = dsdf_ext;
     const long long ntiles = (M + tc::TM - 1) / tc::TM;
     const int sms = nl_num_sms();
-    int grid = (int)(ntiles < (long long)sms ? ntiles : (long long)sms);
-    // NL_TC_PAIR=1: CTA pairs share every weight stage through multicast copies (see k_mlp_tc_train); needs TS and an even grid
-    static const bool use_pair = [] { const char *e = getenv("NL_TC_PAIR"); return e ? atoi(e) != 0 : false; }();
+    const int grid = (int)(ntiles < (long long)sms ? ntiles : (long long)sms);
     static long long *dbg_dev = nullptr;
     static int dbg_calls = 0;
     const bool want_dbg = getenv("NL_TC_TIMELINE") != nullptr;
-    static const int conv_warps = [] { const char *e = getenv("NL_DW_CONV_WARPS"); return (e && atoi(e) == 4) ? 4 : 8; }();   // converter warps of the weight-gradient kernels
-    static const int dw_rings = [] {
-        const char *e = getenv("NL_DW_RINGS");
-        return !e ? 2 : (e[0] == 's' ? 0 : (e[0] == 'm' ? 1 : 2));
-    }();
-    static const bool use_ts = [] { const char *e = getenv("NL_TC_TS"); return e ? atoi(e) != 0 : true; }();   // A operands of the backward GEMMs from TMEM (NL_TC_TS=0: shared memory)
     if (want_dbg && !dbg_dev) { cudaMalloc(&dbg_dev, 4 * 25 * 8 * sizeof(long long)); cudaMemset(dbg_dev, 0, 4 * 25 * 8 * sizeof(long long)); }
     p.dbg = want_dbg ? dbg_dev : nullptr;
     if (grads) {
@@ -1464,9 +1354,7 @@ extern "C" int nl_mlp_tc_train(int64_t M, const int32_t *d_M_dev, const float *f
         p.act_h1 = act; p.act_dh1 = act + panel; p.act_dsdf = act + 2 * panel;
         p.act_mask2 = reinterpret_cast<uint32_t *>(act + 2 * panel + (size_t)ntiles * tc::TM);
         p.gb2 = grads->gb2;
-        if (use_ts && use_pair) { if (int rc = tc::launch_pair(tc::k_mlp_tc_train<true, true, true>, grid, sms, p, stream)) return rc; }
-        else if (use_ts) tc::k_mlp_tc_train<true, true, false><<<grid, tc::NTHREADS_TRAIN, tc::SMEM_TOTAL, stream>>>(p);
-        else tc::k_mlp_tc_train<true, false, false><<<grid, tc::NTHREADS_TRAIN, tc::SMEM_TOTAL, stream>>>(p);
+        tc::k_mlp_tc_train<true><<<grid, tc::NTHREADS_TRAIN, tc::SMEM_TOTAL, stream>>>(p);
         // The weight-gradient kernels only need what the kernel above wrote; on a second stream they overlap with whatever the
         // caller enqueues next on `stream` (the embedding scatter, which is L2-atomic bound and leaves the SMs mostly idle).
         cudaStream_t ws = wgrad_stream_ ? (cudaStream_t)wgrad_stream_ : stream;
@@ -1476,46 +1364,12 @@ extern "C" int nl_mlp_tc_train(int64_t M, const int32_t *d_M_dev, const float *f
             if (cudaEventRecord(ev, stream) != cudaSuccess || cudaStreamWaitEvent(ws, ev, 0) != cudaSuccess)
                 return nl_set_error_code(NL_ERR_CUDA, "nl_mlp_tc_train: could not order the weight-gradient stream behind the decoder kernel");
         }
-        // ring depths (raw, converted): "deep" (4,3)/(4,4) = 219 KB of shared memory per CTA, "mid" (3,3)/(4,3) = 201/183 KB,
-        // "shallow" (3,2)/(3,3) = 149/161 KB -- the smaller ones leave room for blocks of other kernels on the same SM when
-        // the engine pipelines iterations (NL_DW_RINGS)
-        // Experiment kept behind a switch (default off): the two weight-gradient kernels are independent -- k_dw1_tc tensor-bound,
-        // k_dw0_tc streaming 1 KB/sample for a 256x32 result -- so they could run side by side on disjoint SM subsets
-        // (NL_DW_SPLIT = SMs given to k_dw1_tc, the rest to k_dw0_tc on an internal third stream) instead of back to back.
-        // Measured on the B200: slower for every split (100: +0.05 ms ... 126: +0.6 ms per step) -- k_dw0_tc is limited per SM
-        // (its converter warps), not by HBM chip-wide, so it needs all 148 SMs.
-        static const int dw_split = [] { const char *e = getenv("NL_DW_SPLIT"); return e ? atoi(e) : 0; }();
-        const bool split = dw_split > 0 && dw_split < sms - 8;
-        const int sms1 = split ? dw_split : sms, sms0 = split ? sms - dw_split : sms;
-        cudaStream_t ws0 = ws;
-        if (split) {
-            if (!s2_dev[cur_dev] && (cudaStreamCreateWithFlags(&s2_dev[cur_dev], cudaStreamNonBlocking) != cudaSuccess ||
-                                     cudaEventCreateWithFlags(&e2_dev[cur_dev], cudaEventDisableTiming) != cudaSuccess ||
-                                     cudaEventCreateWithFlags(&e3_dev[cur_dev], cudaEventDisableTiming) != cudaSuccess))
-                return nl_set_error_code(NL_ERR_CUDA, "nl_mlp_tc_train: could not create the internal weight-gradient stream");
-            ws0 = s2_dev[cur_dev];
-            if (cudaEventRecord(e2_dev[cur_dev], ws) != cudaSuccess || cudaStreamWaitEvent(ws0, e2_dev[cur_dev], 0) != cudaSuccess)   // fork behind the decoder kernel
-                return nl_set_error_code(NL_ERR_CUDA, "nl_mlp_tc_train: could not fork the internal weight-gradient stream");
-        }
-#define NL_DW_LAUNCH(NCW_, THR, R1, C1, R0, C0)                                                                                     \
-        tc::k_dw1_tc<NCW_, R1, C1><<<sms1, THR, tc::dw_smem(R1, C1), ws>>>(M, d_M_dev, p.act_mask2, p.act_dsdf, p.act_h1, W1, w2, grads->gW1, \
-                                                                            grads->gW2);                                             \
-        tc::k_dw0_tc<NCW_, R0, C0><<<sms0, THR, tc::d0_smem(R0, C0), ws0>>>(M, d_M_dev, p.act_dh1, feats, grads->gW0, grads->gb0);
-        if (conv_warps == 8) {
-            if (dw_rings == 2) { NL_DW_LAUNCH(8, 320, 4, 3, 4, 4) } else if (dw_rings == 1) { NL_DW_LAUNCH(8, 320, 3, 3, 4, 3) } else { NL_DW_LAUNCH(8, 320, 3, 2, 3, 3) }
-        } else {
-            if (dw_rings == 2) { NL_DW_LAUNCH(4, 192, 4, 3, 4, 4) } else if (dw_rings == 1) { NL_DW_LAUNCH(4, 192, 3, 3, 4, 3) } else { NL_DW_LAUNCH(4, 192, 3, 2, 3, 3) }
-        }
-#undef NL_DW_LAUNCH
-        if (split) {      // join: `ws` (what the caller waits on) completes only after k_dw0_tc
-            if (cudaEventRecord(e3_dev[cur_dev], ws0) != cudaSuccess || cudaStreamWaitEvent(ws, e3_dev[cur_dev], 0) != cudaSuccess)
-                return nl_set_error_code(NL_ERR_CUDA, "nl_mlp_tc_train: could not join the internal weight-gradient stream");
-        }
+        // back to back on all SMs: k_dw0_tc streams 1 KB/sample and is limited per SM by its converter warps, so it needs every SM
+        tc::k_dw1_tc<<<sms, tc::DW_THREADS, tc::DW_SMEM, ws>>>(M, d_M_dev, p.act_mask2, p.act_dsdf, p.act_h1, W1, w2, grads->gW1, grads->gW2);
+        tc::k_dw0_tc<<<sms, tc::DW_THREADS, tc::D0_SMEM, ws>>>(M, d_M_dev, p.act_dh1, feats, grads->gW0, grads->gb0);
         tc::k_mask_colsum<<<sms * 8, 256, 0, ws>>>(M, d_M_dev, p.act_mask2, p.act_dsdf, b1, w2, grads->gb1, grads->gW2);
     } else {
-        if (use_ts && use_pair) { if (int rc = tc::launch_pair(tc::k_mlp_tc_train<false, true, true>, grid, sms, p, stream)) return rc; }
-        else if (use_ts) tc::k_mlp_tc_train<false, true, false><<<grid, tc::NTHREADS_TRAIN, tc::SMEM_TOTAL, stream>>>(p);
-        else tc::k_mlp_tc_train<false, false, false><<<grid, tc::NTHREADS_TRAIN, tc::SMEM_TOTAL, stream>>>(p);
+        tc::k_mlp_tc_train<false><<<grid, tc::NTHREADS_TRAIN, tc::SMEM_TOTAL, stream>>>(p);
     }
     NL_CHECK_LAUNCH("nl_mlp_tc_train");
     if (want_dbg && ++dbg_calls == 8) {   // debug only: dump one steady-state tile timeline of CTA 0 (synchronises)

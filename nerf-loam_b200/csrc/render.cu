@@ -14,8 +14,6 @@
 //   k_scan<SAMPLES> : 1 block       exclusive scan of samples per ray -> offsets, M
 //   k_sample<true>  : 1 thread/hit ray  sampler again, writes the compact sample list
 // The reference keeps every intermediate as a padded dense tensor and syncs the host 6 times to size them.
-#include <cstdlib>
-
 #include "loss.cuh"
 #include "sampler.cuh"
 #include "traverse.cuh"
@@ -277,15 +275,14 @@ __global__ void k_pack_children(int n_nodes, const int32_t *__restrict__ ids, co
 // ------------------------------------------------------------------------------------------------
 enum { SCAN_HITS = 0, SCAN_SAMPLES = 1 };
 
-template <int MODE, bool STAGE = true>   // STAGE = false: no shared-memory staging of the compacted ray list (the block then needs 256 B of
-                                          // shared memory and can share an SM with the persistent weight-gradient CTAs of the previous iteration)
+template <int MODE>
 __global__ void __launch_bounds__(1024) k_scan(int n, const int32_t *__restrict__ in, int32_t *__restrict__ out,
                                                 int32_t *__restrict__ hitray, nl_render_stats *stats, int sample_capacity) {
     // tiles of 4096 elements: every thread owns 4 consecutive ones (one 16-byte load, issued one tile ahead so that its
     // latency hides behind the previous tile), warp shuffle scan, then every warp scans the 32 warp totals redundantly:
     // one __syncthreads per tile (the totals are double-buffered) and the running carry stays in registers
     __shared__ int wsum[2][32];
-    __shared__ int compact[(MODE == SCAN_HITS && STAGE) ? 4096 : 1];
+    __shared__ int compact[MODE == SCAN_HITS ? 4096 : 1];
     const int t = threadIdx.x, lane = t & 31, w = t >> 5;
     auto load4 = [&](int i0) {
         int4 x = make_int4(0, 0, 0, 0);
@@ -343,25 +340,16 @@ __global__ void __launch_bounds__(1024) k_scan(int n, const int32_t *__restrict_
                 if (i0 + 1 < n) out[i0 + 1] = o.y;
                 if (i0 + 2 < n) out[i0 + 2] = o.z;
             }
-            if (STAGE) {
-                int loc = run - carry;
+            int loc = run - carry;
 #pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    if (v[k]) compact[loc] = i0 + k;     // v[k] is 0 for i0 + k >= n
-                    loc += v[k];
-                }
-                __syncthreads();
-                for (int j = t; j < tile_total; j += 1024) hitray[carry + j] = compact[j];
-                // the next tile's writes to compact[] come after its own __syncthreads (warp totals), which every thread reaches
-                // only after finishing this copy
-            } else {
-                int loc = run;                            // positions ascend with the thread index: a warp's writes fall into one short range
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    if (v[k]) hitray[loc] = i0 + k;
-                    loc += v[k];
-                }
+            for (int k = 0; k < 4; ++k) {
+                if (v[k]) compact[loc] = i0 + k;     // v[k] is 0 for i0 + k >= n
+                loc += v[k];
             }
+            __syncthreads();
+            for (int j = t; j < tile_total; j += 1024) hitray[carry + j] = compact[j];
+            // the next tile's writes to compact[] come after its own __syncthreads (warp totals), which every thread reaches
+            // only after finishing this copy
         } else {
             const int4 o = make_int4(run, run + v[0], run + v[0] + v[1], run + v[0] + v[1] + v[2]);
             if (i0 + 3 < n) {
@@ -841,10 +829,8 @@ extern "C" int nl_render_samples(const nl_render_args *a, void *stream_) {
     const int blocks = nl_div_up(R, 128);
     // lanes per ray: 8 (one per child) while the launch is latency-bound -- a tracking / real-size mapping iteration has 2-10 k rays,
     // far fewer than the GPU holds threads for (B200: 5.99 -> 5.53 ms per 25-iteration scan, 15.8 -> 15.2 ms per 5-frame mapping call);
-    // 4 once the rays alone fill the SMs (83 k rays: 1.575 vs 1.617 ms per step).  NL_TRAVERSE_LANES=4|8 overrides.
-    static const int co_lanes_env = [] { const char *e = getenv("NL_TRAVERSE_LANES"); return e ? atoi(e) : 0; }();
-    const int co_lanes = (co_lanes_env == 4 || co_lanes_env == 8) ? co_lanes_env : (R <= 32768 ? 8 : 4);
-    if (a->d_packed_children && co_lanes == 8)
+    // 4 once the rays alone fill the SMs (83 k rays: 1.575 vs 1.617 ms per step).
+    if (a->d_packed_children && R <= 32768)
         k_traverse_coop<8><<<nl_div_up(R, 32), 256, 0, stream>>>(R, a->voxel_size, a->max_distance, a->d_centres, a->d_structure,
                                                                   (const float4 *)a->d_packed_children, a->d_ray_o, a->d_ray_d, ws,
                                                                   a->d_ray_nsamp, a->d_stats);
@@ -855,17 +841,15 @@ extern "C" int nl_render_samples(const nl_render_args *a, void *stream_) {
     else
         k_traverse_sort<<<nl_div_up(R, 64), 64, 0, stream>>>(R, a->voxel_size, a->max_distance, a->d_centres, a->d_structure, a->d_ray_o,
                                                               a->d_ray_d, ws, a->d_ray_nsamp, a->d_stats);
-    // NL_SCAN_STAGE=0: the hit scan without its 16 KB staging buffer (see k_scan)
-    static const bool scan_stage = [] { const char *e = getenv("NL_SCAN_STAGE"); return e ? atoi(e) != 0 : true; }();
-    // NL_SCAN=single: the single-block scans (the fallback for more than 4 M rays)
-    static const bool scan_chained = [] { const char *e = getenv("NL_SCAN"); return !(e && e[0] == 's'); }();
+    // the single-block scans are the fallback for more than 4 M rays
     const int scan_tiles = nl_div_up(R, 4096);
-    const bool chained = scan_chained && scan_tiles <= SCAN_MAX_TILES;
+    const bool chained = scan_tiles <= SCAN_MAX_TILES;
     if (chained) {
         cudaMemsetAsync(ws.scan, 0, sizeof(unsigned long long) * 2 * SCAN_SCRATCH, stream);
         k_scan_chained<SCAN_HITS><<<scan_tiles, 1024, 0, stream>>>(R, ws.nvalid, a->d_hit_rank, ws.hitray, a->d_stats, 0, ws.scan);
-    } else if (scan_stage) k_scan<SCAN_HITS, true><<<1, 1024, 0, stream>>>(R, ws.nvalid, a->d_hit_rank, ws.hitray, a->d_stats, 0);
-    else k_scan<SCAN_HITS, false><<<1, 1024, 0, stream>>>(R, ws.nvalid, a->d_hit_rank, ws.hitray, a->d_stats, 0);
+    } else {
+        k_scan<SCAN_HITS><<<1, 1024, 0, stream>>>(R, ws.nvalid, a->d_hit_rank, ws.hitray, a->d_stats, 0);
+    }
     SampleParams p;
     p.R = R; p.sample_capacity = a->sample_capacity; p.compat = a->reference_compat;
     p.step_size = a->step_size; p.truncation = a->truncation; p.max_depth = a->max_depth;

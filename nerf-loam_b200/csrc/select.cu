@@ -24,13 +24,13 @@ __device__ __forceinline__ uint32_t point_key(uint32_t seed, uint32_t i) { retur
 
 constexpr int SEL_THREADS = 1024;
 constexpr int SEL_BINS = 2048;
-constexpr int SEL_CLUSTER = 8;
-constexpr int SEL_KEYS = 16;        // keys a thread keeps in registers between the passes (covers scans of up to 8 x 1024 x 16 = 131 072 points)      // CTAs per scan: each hashes an eighth of the points, histograms are summed over distributed shared memory
+constexpr int SEL_CLUSTER = 8;     // CTAs per scan: each hashes an eighth of the points, histograms are summed over distributed shared memory
+constexpr int SEL_KEYS = 16;        // keys a thread keeps in registers between the passes (covers scans of up to 8 x 1024 x 16 = 131 072 points)
 
 // Among this scan's keys that pass `match`, find the bin (of `digit`) in which the `want`-th smallest key (1-based) lies, and the
 // number of matching keys in lower bins.  Every CTA of the cluster histograms its own points [p0, p1), reads the other CTAs'
 // histograms through DSMEM and finds the bin redundantly.  hist: SEL_BINS ints of shared memory (same offset in every CTA).
-template <int CL, class Match, class Digit>
+template <class Match, class Digit>
 __device__ void find_bin(cg::cluster_group &cluster, int p0, int p1, uint32_t seed, const uint32_t (&keys)[SEL_KEYS], bool cached, int want, Match match,
                          Digit digit, int *hist, int *s_scan, int &bin, int &below) {
     const int t = threadIdx.x;
@@ -49,7 +49,7 @@ __device__ void find_bin(cg::cluster_group &cluster, int p0, int p1, uint32_t se
     cluster.sync();
     int a = 0, b = 0;
 #pragma unroll
-    for (int q = 0; q < CL; ++q) {
+    for (int q = 0; q < SEL_CLUSTER; ++q) {
         const int2 h = *reinterpret_cast<const int2 *>(cluster.map_shared_rank(hist, q) + 2 * t);
         a += h.x; b += h.y;
     }
@@ -76,7 +76,6 @@ __device__ void find_bin(cg::cluster_group &cluster, int p0, int p1, uint32_t se
     // (no cluster barrier here: every pass has its own histogram, so a CTA may start the next pass while a peer still reads this one)
 }
 
-template <int CL>
 __global__ void __launch_bounds__(SEL_THREADS)
     k_select_rays(int cap, int n_select, const int64_t *__restrict__ n_points, const uint32_t *__restrict__ seed_dev, uint32_t seed_host,
                   const float *__restrict__ dirs_all, const float *__restrict__ gt_all, const float *__restrict__ cos_all, float *__restrict__ dirs,
@@ -86,13 +85,13 @@ __global__ void __launch_bounds__(SEL_THREADS)
     __shared__ unsigned long long s_w[SEL_THREADS / 32];
     __shared__ unsigned long long s_total;
     cg::cluster_group cluster = cg::this_cluster();
-    const int f = blockIdx.x / CL, c = (int)cluster.block_rank(), t = threadIdx.x, lane = t & 31, w = t >> 5;
+    const int f = blockIdx.x / SEL_CLUSTER, c = (int)cluster.block_rank(), t = threadIdx.x, lane = t & 31, w = t >> 5;
     const int n = (int)min((long long)n_points[f], (long long)cap);
     const int N = min(n_select, n);
     uint32_t seed = seed_dev ? *seed_dev : seed_host;
     seed = mix32(seed ^ 0x9E3779B9u * (uint32_t)(f + 1));
     // this CTA's contiguous share of the scan, and inside it every thread's contiguous run (for the ordered emission)
-    const int share = (n + CL - 1) / CL;
+    const int share = (n + SEL_CLUSTER - 1) / SEL_CLUSTER;
     const int c0 = min(c * share, n), c1 = min(c0 + share, n);
     // threshold key T = the N-th smallest key; `ties` = how many of the keys equal to T belong to the N smallest
     uint32_t T = 0xffffffffu;
@@ -109,13 +108,13 @@ __global__ void __launch_bounds__(SEL_THREADS)
     }
     if (N < n && N > 0) {
         int bA, bB, bC, below;
-        find_bin<CL>(cluster, c0, c1, seed, keys, cached, N, [](uint32_t) { return true; }, [](uint32_t k) { return (int)(k >> 21); }, hist[0], s_scan, bA, below);
+        find_bin(cluster, c0, c1, seed, keys, cached, N, [](uint32_t) { return true; }, [](uint32_t k) { return (int)(k >> 21); }, hist[0], s_scan, bA, below);
         int want = N - below;
-        find_bin<CL>(cluster, c0, c1, seed, keys, cached, want, [bA](uint32_t k) { return (int)(k >> 21) == bA; }, [](uint32_t k) { return (int)((k >> 10) & 2047u); }, hist[1],
+        find_bin(cluster, c0, c1, seed, keys, cached, want, [bA](uint32_t k) { return (int)(k >> 21) == bA; }, [](uint32_t k) { return (int)((k >> 10) & 2047u); }, hist[1],
                  s_scan, bB, below);
         want -= below;
         const uint32_t top22 = ((uint32_t)bA << 11) | (uint32_t)bB;
-        find_bin<CL>(cluster, c0, c1, seed, keys, cached, want, [top22](uint32_t k) { return (k >> 10) == top22; }, [](uint32_t k) { return (int)(k & 1023u); }, hist[2], s_scan,
+        find_bin(cluster, c0, c1, seed, keys, cached, want, [top22](uint32_t k) { return (k >> 10) == top22; }, [](uint32_t k) { return (int)(k & 1023u); }, hist[2], s_scan,
                  bC, below);
         T = (top22 << 10) | (uint32_t)bC;
         ties = want - below;
@@ -169,23 +168,17 @@ extern "C" int nl_select_rays(int n_frames, int cap, int n_select, const int64_t
                               int32_t *d_idx, void *stream) {
     if (n_frames <= 0 || cap <= 0 || n_select <= 0) return nl_set_error("nl_select_rays: sizes must be positive");
     if (!d_n_points || !d_dirs_all || !d_gt_all || !d_cos_all || !d_dirs || !d_gt || !d_cos) return nl_set_error("nl_select_rays: null pointer");
-    static const bool single = [] { const char *e = getenv("NL_SEL_CLUSTER"); return e && e[0] == '0'; }();
-    if (single) {
-        k_select_rays<1><<<n_frames, SEL_THREADS, 0, (cudaStream_t)stream>>>(cap, n_select, d_n_points, d_seed, seed, d_dirs_all, d_gt_all, d_cos_all,
-                                                                                d_dirs, d_gt, d_cos, d_idx);
-    } else {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(n_frames * SEL_CLUSTER);
-        cfg.blockDim = dim3(SEL_THREADS);
-        cfg.stream = (cudaStream_t)stream;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = SEL_CLUSTER; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        const cudaError_t e = cudaLaunchKernelEx(&cfg, k_select_rays<SEL_CLUSTER>, cap, n_select, d_n_points, d_seed, seed, d_dirs_all, d_gt_all, d_cos_all,
-                                                 d_dirs, d_gt, d_cos, d_idx);
-        if (e != cudaSuccess) return nl_set_error_code(NL_ERR_CUDA, cudaGetErrorString(e));
-    }
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(n_frames * SEL_CLUSTER);
+    cfg.blockDim = dim3(SEL_THREADS);
+    cfg.stream = (cudaStream_t)stream;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = SEL_CLUSTER; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, k_select_rays, cap, n_select, d_n_points, d_seed, seed, d_dirs_all, d_gt_all, d_cos_all,
+                                             d_dirs, d_gt, d_cos, d_idx);
+    if (e != cudaSuccess) return nl_set_error_code(NL_ERR_CUDA, cudaGetErrorString(e));
     NL_CHECK_LAUNCH("nl_select_rays");
     return NL_OK;
 }

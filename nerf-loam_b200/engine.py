@@ -281,9 +281,9 @@ class SDFEngine:
         self._stats_host = torch.empty(STATS_BYTES, dtype=torch.uint8).pin_memory() if torch.cuda.is_available() else None
         self.events = None            # set to {} to record CUDA events around the main kernels (bench.py)
         # the weight-gradient kernels of the decoder run on a second stream, concurrently with the embedding scatter
-        self.overlap_wgrad = os.environ.get("NL_OVERLAP_WGRAD", "1") != "0"
+        self.overlap_wgrad = True
         # warp-cooperative traversal over the packed octree image; False: one thread per ray over (centres, structure)
-        self.use_packed_octree = os.environ.get("NL_PACKED_OCTREE", "1") != "0"
+        self.use_packed_octree = True
         self._side = None
         # software pipelining across iterations (forward_backward(defer_wgrad=True)): the weight-gradient kernels and the decoder's
         # Adam of iteration i stay on the side stream while the main stream already runs the embedding scatter, the other Adam

@@ -533,7 +533,7 @@ def bundle_adjust_frames(keyframe_graph, embeddings, map_states, sdf_network, lo
         return eng.read_ctl()
 
     graph_ok = ray_selection == "device" and noise_per_iter is None and loss_log is None and \
-        all(f.points.shape[0] >= N_rays for f in frames) and os.environ.get("NL_MAP_GRAPH", "1") != "0"
+        all(f.points.shape[0] >= N_rays for f in frames)
     if cuda_graph is None:
         # automatic only for maps whose arrays keep their addresses across map updates (mapping.MapUpdater): a capture costs about
         # as much as 1.5 eager calls, so re-capturing for every new map (the reference's per-frame dicts) would be a net loss
@@ -715,7 +715,7 @@ def track_frame(frame_pose, curr_frame, map_states, sdf_network, loss_criteria, 
     graph_ok = ray_selection == "device" and noise_per_iter is None and loss_log is None and curr_frame.points.shape[0] >= N_rays
     if cuda_graph is None:          # default: the captured path for maps with stable addresses (mapping.MapUpdater), see bundle_adjust_frames
         stable = getattr(map_states, "stable", False) or getattr(map_states.get("_mapstate") if isinstance(map_states, dict) else None, "stable", False)
-        cuda_graph = graph_ok and stable and os.environ.get("NL_TRACK_GRAPH", "1") != "0"
+        cuda_graph = graph_ok and stable
     if cuda_graph:
         if not graph_ok:
             raise ValueError("cuda_graph=True needs ray_selection='device', no per-iteration host inputs/outputs and >= N_rays points")

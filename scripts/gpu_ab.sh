@@ -1,6 +1,6 @@
 #!/bin/bash
 # A/B visit: for every variant "NAME:ENV=VAL,ENV=VAL" run the GPU suite (first variant: whole suite; others: -x) and a short bench.
-# usage: gpu_ab.sh TAG "base:" "merge:NL_GATHER_MERGE=1" ...
+# usage: gpu_ab.sh TAG "base:" "nopipe:NL_PIPELINE=0" ...
 tag=$1; shift; out=gpurun_out/$tag; mkdir -p $out
 export NL_BENCH_SKIP_CPU=1
 for spec in "$@"; do
